@@ -27,6 +27,10 @@ strong_2p30  configs[2]: global N = 2^30 sharded over the N ranks (2^30/N per GP
 cli_strong_2p30  the same shape through the C++ executable's one-thread-per-GPU path (`vectorAdd --gpus N`),
              run by rank 0 on exactly the GPUs the ranks drove
 loop_2p24    configs[4]: 5000 launches of N = 2^24 in 50-launch CUDA graphs on each GPU
+
+--dump-outputs DIR writes what the last timed step returned -- a fixed, seeded sample of C --
+so that two builds run with the same arguments (hence the same inputs) can be compared
+element for element (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -54,6 +58,7 @@ DIGEST_2P30 = (0x0FD8E36879AED49F, 0x0F23C595)
 DIGEST_2P24 = (0x003F639456AC9687, 0x064A9499)
 READ_ONLY_CEILING_GBPS = 7436.0   # pure read stream (A and B in, nothing out) with the production geometry: profiles/r02/a_channel_skew.jsonl
 LINK_ALONE_MS_PER_2P28 = 40.8   # one GPU's PCIe Gen5 x16 link, 2 GiB in + 1 GiB out concurrently (profiles/r01/l_pcie_probe.jsonl)
+DUMP_SAMPLE = 1 << 22   # elements of C drawn for --dump-outputs over all ranks: 16 MiB of values + 32 MiB of indices
 
 
 # --------------------------------------------------------------------------- clocks
@@ -162,8 +167,7 @@ def run_reference(args) -> None:
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
-    steps = min(steps, 50)  # 2^28 elements per pass on host cores: keep the run within minutes
+    steps, warmup = args.steps, args.warmup
     cb = cpu_baseline_line(N_PER_GPU, warmup, steps)
     total = sum(cb.pop("secs"))
     value = cb["value"]
@@ -302,6 +306,21 @@ def cli_strong(gpus: int, cli: str, devices: list[int] | None = None) -> dict:
             "digest_ok": (int(r["digest_sum"], 16), int(r["digest_xor"], 16)) == DIGEST_2P30}
 
 
+def dump_outputs(out_dir: str, c, first: int, rank: int, ws: int) -> None:
+    """Writes a sample of this rank's C as <out_dir>/c_rank<r>.npy (float32) and the global element
+    index of every sampled value as <out_dir>/index_rank<r>.npy (float64, exact below 2^53).  The
+    indices are drawn from a generator seeded with the rank, so they only depend on the shard size."""
+    import numpy as np
+    import torch
+
+    rng = np.random.default_rng(rank)
+    idx = np.unique(rng.integers(0, c.numel(), min(c.numel(), DUMP_SAMPLE // ws)))
+    vals = c[torch.from_numpy(idx).to(c.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"c_rank{rank}.npy"), vals.astype(np.float32))
+    np.save(os.path.join(out_dir, f"index_rank{rank}.npy"), (idx + first).astype(np.float64))
+
+
 def run_ours(args, emit=print) -> None:
     import torch
 
@@ -353,6 +372,8 @@ def run_ours(args, emit=print) -> None:
     bad, first_bad = va.verify(a, b, c)
     bad_total = int(sharding.sum_over_ranks(bad))
     dig = sharding.combine_digests(va.digest(c))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, c, first, rank, ws)      # before the loop leg below rewrites c[:2^24]
 
     # ---- the ceiling, live: the same launch geometry with the stores removed (a pure read stream of A and B)
     for _ in range(3):
@@ -608,8 +629,13 @@ def main() -> None:
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip strong_2p30 and loop_2p24")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's C to DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl ours")
         run_reference(args)
         return
     try:

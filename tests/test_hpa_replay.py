@@ -7,16 +7,16 @@ from conftest import ROOT
 from k8s_gpu_hpa_b200 import hpa_replay as hr
 
 
-def test_constants_match_the_reference_manifests_when_present():
-    ref = "/root/reference"
-    if not os.path.isdir(ref):
-        pytest.skip("reference tree not present on this machine")
-    hpa = open(os.path.join(ref, "cuda-test-hpa.yaml")).read()
-    assert f"targetValue: {int(hr.HPA_TARGET)}" in hpa
-    assert f"minReplicas: {hr.HPA_MIN}" in hpa and f"maxReplicas: {hr.HPA_MAX}" in hpa
-    assert f'"-c", "{int(hr.DCGM_INTERVAL_S * 1000)}"' in open(os.path.join(ref, "dcgm-exporter.yaml")).read().replace("'", '"') \
-        or "10000" in open(os.path.join(ref, "dcgm-exporter.yaml")).read()
-    assert "scrape_interval: 1s" in open(os.path.join(ref, "kube-prometheus-stack-values.yaml")).read()
+def test_constants_match_the_reference_manifests():
+    """The values the reference's manifests set, as extracted by tests/golden/make_reference_manifests.py."""
+    import json
+
+    ref = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_manifests.json")))
+    assert hr.HPA_TARGET == ref["hpa_target_value"]
+    assert (hr.HPA_MIN, hr.HPA_MAX) == (ref["hpa_min_replicas"], ref["hpa_max_replicas"])
+    assert ref["hpa_metric"] == hr.cuda_test_gpu_avg.__name__
+    assert hr.DCGM_INTERVAL_S * 1000 == ref["dcgm_collect_interval_ms"]
+    assert f"{hr.SCRAPE_INTERVAL_S:g}s" == ref["scrape_interval"]
 
 
 def test_recording_rule_max_by_pod_then_avg_over_labelled_pods():

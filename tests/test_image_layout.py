@@ -29,15 +29,23 @@ def dockerfile_runtime_copies() -> tuple[str, list[str]]:
     return workdir, [os.path.basename(p) for p in copy]
 
 
-def test_fixture_matches_the_reference_yaml_when_present():
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("reference tree not present on this machine")
+def test_extractor_reads_the_fixture_back_from_a_deployment(tmp_path):
+    """The script that wrote the fixture from the reference's Deployment recovers exactly the
+    fixture from a Deployment whose container carries its values."""
     import importlib.util
+
+    import yaml
 
     spec = importlib.util.spec_from_file_location("mk", os.path.join(os.path.dirname(GOLD), "make_reference_command.py"))
     mk = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mk)
-    assert mk.parse() == reference_command()
+    ref = reference_command()
+    container = {"name": ref["container"], "image": ref["image"], "command": ref["command"],
+                 "resources": {"limits": {"nvidia.com/gpu": ref["gpu_limit"]}}}
+    path = tmp_path / "cuda-test-deployment.yaml"
+    path.write_text(yaml.safe_dump({"apiVersion": "apps/v1", "kind": "Deployment", "metadata": {"name": "cuda-test"},
+                                    "spec": {"template": {"spec": {"containers": [container]}}}}))
+    assert mk.parse(str(path)) == ref
 
 
 def test_reference_command_is_the_bash_loop_over_a_zero_argument_binary():

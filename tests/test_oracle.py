@@ -176,18 +176,17 @@ def test_on_disk_nvidia_derivative_carries_the_restated_float_recipe():
     """The toolkit ships an NVIDIA derivative of the vectorAdd sample with FLOAT operands
     (CUPTI samples, cuda_memory_trace/memory_trace.cu).  It is not the reference's image, but it
     corroborates what oracle/vadd_oracle.c restates from recollection: the kernel body, the
-    interleaved never-seeded rand()/(float)RAND_MAX fill, 256-thread blocks."""
+    interleaved never-seeded rand()/(float)RAND_MAX fill, 256-thread blocks.  Its cited lines are
+    recorded in golden/cupti_memory_trace_recipe.json (tests/golden/make_cupti_recipe.py)."""
     import re
 
-    path = "/usr/local/cuda/extras/CUPTI/samples/cuda_memory_trace/memory_trace.cu"
-    if not os.path.exists(path):
-        pytest.skip("CUPTI samples not installed on this machine")
-    src = open(path).read()
+    g = json.load(open(os.path.join(GOLD, "cupti_memory_trace_recipe.json")))
+    src = "\n".join(g["lines"][k] for k in sorted(g["lines"], key=int))
     flat = re.sub(r"\s+", " ", src)
     assert re.search(r"VectorAdd\( const float \*pA, const float \*pB, float \*pC, int N\)", flat)
     assert "int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < N) { pC[i] = pA[i] + pB[i]; }" in flat
     assert "pHostA[n] = rand() / (float)RAND_MAX; pHostB[n] = rand() / (float)RAND_MAX;" in flat      # A then B, per index
-    assert "srand" not in src                                                                           # glibc default seed 1
+    assert not g["calls_srand"] and "srand" not in src                                                  # glibc default seed 1
     assert "dim3 block(256);" in src
     # ... and that recipe, run through the oracle, is the one whose known answers are pinned above
     a, b = oracle.fill_rand(4)
