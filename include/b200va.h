@@ -267,6 +267,33 @@ int b200va_device_numa_node_of(int device);
 int b200va_stream(int op, int dtype, const void *dA, const void *dB, void *dC, size_t n,
                   double scalar, void *stream);
 
+/* Grouped form: one op and dtype over many independent vectors, in as few launches as the
+ * kernel parameter block allows (800 items per launch; larger calls are split at item
+ * boundaries into launches enqueued in order on `stream`).  Many small vectors then cost one
+ * launch boundary instead of one each -- the torch._foreach_* / multi-tensor-apply shape.
+ *   - Each item's result is bit-identical to  b200va_stream(op, dtype, a, b, c, n, scalar, stream).
+ *   - Asynchronous on `stream`, current device; no hidden allocation or synchronisation, so the
+ *     call can be captured into a CUDA graph.  `items` is host memory, read before the call
+ *     returns: the caller may reuse the array at once.
+ *   - Every item is checked before anything is enqueued, with the checks of b200va_stream
+ *     (NULL with n > 0 or n > 2^40: ERR_INVALID; not aligned to the element size: ERR_ALIGN;
+ *     C partially overlapping its own A or B: ERR_OVERLAP, exact aliasing is fine).  On a
+ *     failure nothing is enqueued and the first failing item's code is returned.
+ *   - count == 0 is a no-op; items == NULL with count > 0 is ERR_INVALID; an unknown op or
+ *     dtype is ERR_VARIANT.  Items with n == 0 are skipped (their pointers may be NULL).
+ *   - PRECONDITION, not checked: items are independent -- no item's C overlaps another item's
+ *     A, B or C.  Items run concurrently in no defined order.  (Checking this needs a sort of
+ *     the address ranges, tens of microseconds of host time per call: more than the GPU time
+ *     of a small batch.) */
+typedef struct b200va_item {
+    const void *a;      /* input A (device)                                       */
+    const void *b;      /* input B (device); ignored, may be NULL, for COPY/SCALE */
+    void       *c;      /* output C (device)                                      */
+    size_t      n;      /* elements; 0 = skipped (pointers may then be NULL)      */
+} b200va_item_t;
+int b200va_stream_grouped(int op, int dtype, const b200va_item_t *items, size_t count,
+                          double scalar, void *stream);
+
 /* ---- ceiling probes (measurement aids; not part of the reference's surface) -------------
  * The production launch geometry with one side of the add's traffic removed, so a harness can
  * measure on the spot what the HBM gives each kind of stream (bench.py reports the add as a

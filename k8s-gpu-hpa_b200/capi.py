@@ -66,6 +66,11 @@ class DevInfo(C.Structure):
                 ("name", C.c_char * 64)]
 
 
+class Item(C.Structure):
+    """b200va_item_t: one (A, B, C, n) item of b200va_stream_grouped."""
+    _fields_ = [("a", C.c_void_p), ("b", C.c_void_p), ("c", C.c_void_p), ("n", C.c_size_t)]
+
+
 if not os.path.exists(LIB_PATH):
     raise ImportError(
         f"{LIB_PATH} is missing: build it with `make -C {_HERE}` (or __graft_entry__.build()). "
@@ -108,6 +113,7 @@ _SIGS = {
     "b200va_device_numa_node": (_I, []),
     "b200va_device_numa_node_of": (_I, [_I]),
     "b200va_stream": (_I, [_I, _I, _P, _P, _P, _SZ, C.c_double, _P]),
+    "b200va_stream_grouped": (_I, [_I, _I, C.POINTER(Item), _SZ, C.c_double, _P]),
     "b200va_probe_f32": (_I, [_I, _P, _P, _P, _SZ, _P]),
     "b200va_shard_range": (_I, [_SZ, _I, _I, C.POINTER(_SZ), C.POINTER(_SZ)]),
 }

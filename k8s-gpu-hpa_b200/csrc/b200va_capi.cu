@@ -627,6 +627,104 @@ int launch_stream_op(int op, const void* dA, const void* dB, void* dC, size_t n,
     return B200VA_ERR_VARIANT;
 }
 
+// ----------------------------------------------------------------------- grouped dispatch
+// Items per launch: the parameter block holds kGroupedCap items of 40 B (record + tile prefix),
+// 32,032 B in all, under the 32,764-B limit of cudaLaunchKernelEx.
+constexpr int kGroupedCap = 800;
+static_assert(sizeof(GroupedParams<kGroupedCap>) + sizeof(double) + sizeof(int) <= 32764, "kernel parameter block too large");
+// Production geometry (threads x unroll per tile) for every op and dtype.
+constexpr unsigned kGroupedThreads = 256;
+constexpr int kGroupedUnroll = 2;
+
+// The checks of b200va_stream, for one item.
+int check_stream_item(const b200va_item_t& it, bool binary, size_t es)
+{
+    if (it.n == 0) return B200VA_OK;
+    if (!it.a || !it.c || (binary && !it.b)) return B200VA_ERR_INVALID;
+    const uintptr_t a = reinterpret_cast<uintptr_t>(it.a), b = reinterpret_cast<uintptr_t>(it.b),
+                    c = reinterpret_cast<uintptr_t>(it.c);
+    if (((a | c | (binary ? b : 0)) & (es - 1)) != 0) return B200VA_ERR_ALIGN;
+    if (it.n > (size_t{1} << 40)) return B200VA_ERR_INVALID;
+    const uintptr_t bytes = it.n * es;
+    auto partial = [&](uintptr_t x) { return x != c && x < c + bytes && c < x + bytes; };
+    if (partial(a) || (binary && partial(b))) return B200VA_ERR_OVERLAP;
+    return B200VA_OK;
+}
+
+// Packs the non-empty items into parameter blocks of CAP, computes each block's tile prefix and
+// launches it; blocks go out in item order on `st`.
+template <int DT, int OP, int UNROLL, int CAP>
+int launch_grouped_blocks(const b200va_item_t* items, size_t count, double scalar, unsigned threads, cudaStream_t st)
+{
+    using S = typename dt_traits<DT>::scalar;
+    constexpr int ES = dt_traits<DT>::size;
+    constexpr bool binary = (OP == OP_ADD || OP == OP_TRIAD);
+    const S s = static_cast<S>(scalar);
+    const size_t tile_vecs = static_cast<size_t>(threads) * UNROLL;
+    GroupedParams<CAP> p;
+    size_t i = 0;
+    while (i < count) {
+        int k = 0;
+        unsigned long long tiles = 0;
+        size_t bytes = 0;
+        for (; i < count && k < CAP; ++i) {
+            const b200va_item_t& it = items[i];
+            if (it.n == 0) continue;
+            p.item[k] = GroupedItem{it.a, it.b, it.c, it.n};
+            p.first_tile[k] = tiles;
+            tiles += grouped_shape<ES, binary>(it.a, it.b, it.c, it.n, tile_vecs).ntiles;
+            bytes += it.n * ES;
+            ++k;
+        }
+        if (k == 0) break;
+        p.count = k;
+        p.total_tiles = tiles;
+        const unsigned grid = static_cast<unsigned>(tiles > 0x7fffffffull ? 0x7fffffffull : tiles);   // the kernel loops tile += gridDim.x
+        const int prefetch_first = bytes >= (size_t{1} << 27) ? 1 : 0;     // >= 128 MiB per array: never L2-resident
+        RC_TRY(launch_kernel(stream_grouped<DT, OP, UNROLL, CAP>, grid, threads, 0, st, p, s, prefetch_first));
+    }
+    return B200VA_OK;
+}
+
+template <int DT, int OP>
+int launch_grouped_typed(const b200va_item_t* items, size_t count, double scalar, cudaStream_t st)
+{
+#ifdef B200VA_TUNE_MATRIX
+    // development knob for profiles/ (tune library only): B200VA_GROUPED_GEOMETRY="threads,unroll,capacity",
+    // unroll 1 | 2 | 4, capacity 100 | 800
+    static const struct Override { int threads = 0, unroll = 0, cap = 0; } ov = [] {
+        Override o;
+        if (const char* e = std::getenv("B200VA_GROUPED_GEOMETRY")) std::sscanf(e, "%d,%d,%d", &o.threads, &o.unroll, &o.cap);
+        return o;
+    }();
+    if (ov.threads >= 32 && ov.threads <= 1024 && (ov.threads & 31) == 0 && (ov.cap == 100 || ov.cap == kGroupedCap)) {
+        const unsigned t = static_cast<unsigned>(ov.threads);
+        if (ov.cap == 100) {
+            if (ov.unroll == 1) return launch_grouped_blocks<DT, OP, 1, 100>(items, count, scalar, t, st);
+            if (ov.unroll == 2) return launch_grouped_blocks<DT, OP, 2, 100>(items, count, scalar, t, st);
+            if (ov.unroll == 4) return launch_grouped_blocks<DT, OP, 4, 100>(items, count, scalar, t, st);
+        } else {
+            if (ov.unroll == 1) return launch_grouped_blocks<DT, OP, 1, kGroupedCap>(items, count, scalar, t, st);
+            if (ov.unroll == 2) return launch_grouped_blocks<DT, OP, 2, kGroupedCap>(items, count, scalar, t, st);
+            if (ov.unroll == 4) return launch_grouped_blocks<DT, OP, 4, kGroupedCap>(items, count, scalar, t, st);
+        }
+    }
+#endif
+    return launch_grouped_blocks<DT, OP, kGroupedUnroll, kGroupedCap>(items, count, scalar, kGroupedThreads, st);
+}
+
+template <int DT>
+int launch_grouped_op(int op, const b200va_item_t* items, size_t count, double scalar, cudaStream_t st)
+{
+    switch (op) {
+        case OP_COPY:  return launch_grouped_typed<DT, OP_COPY>(items, count, scalar, st);
+        case OP_SCALE: return launch_grouped_typed<DT, OP_SCALE>(items, count, scalar, st);
+        case OP_ADD:   return launch_grouped_typed<DT, OP_ADD>(items, count, scalar, st);
+        case OP_TRIAD: return launch_grouped_typed<DT, OP_TRIAD>(items, count, scalar, st);
+    }
+    return B200VA_ERR_VARIANT;
+}
+
 }  // namespace
 
 // =============================================================================== ABI
@@ -961,6 +1059,26 @@ int b200va_stream(int op, int dtype, const void* dA, const void* dB, void* dC, s
         case DT_F64:  return launch_stream_op<DT_F64>(op, dA, dB, dC, n, scalar, st);
         case DT_F16:  return launch_stream_op<DT_F16>(op, dA, dB, dC, n, scalar, st);
         case DT_BF16: return launch_stream_op<DT_BF16>(op, dA, dB, dC, n, scalar, st);
+    }
+    return B200VA_ERR_VARIANT;
+}
+
+int b200va_stream_grouped(int op, int dtype, const b200va_item_t* items, size_t count, double scalar, void* stream)
+{
+    if (op < 0 || op >= OP_COUNT || dtype < 0 || dtype >= DT_COUNT) return B200VA_ERR_VARIANT;
+    const b200va_devinfo_t* di = nullptr;
+    RC_TRY(current_dev_info(&di));
+    if (count == 0) return B200VA_OK;
+    if (!items) return B200VA_ERR_INVALID;
+    const bool binary = (op == OP_ADD || op == OP_TRIAD);
+    const size_t es = dtype == DT_F64 ? 8 : dtype == DT_F32 ? 4 : 2;
+    for (size_t i = 0; i < count; ++i) RC_TRY(check_stream_item(items[i], binary, es));   // nothing is enqueued on a failure
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    switch (dtype) {
+        case DT_F32:  return launch_grouped_op<DT_F32>(op, items, count, scalar, st);
+        case DT_F64:  return launch_grouped_op<DT_F64>(op, items, count, scalar, st);
+        case DT_F16:  return launch_grouped_op<DT_F16>(op, items, count, scalar, st);
+        case DT_BF16: return launch_grouped_op<DT_BF16>(op, items, count, scalar, st);
     }
     return B200VA_ERR_VARIANT;
 }

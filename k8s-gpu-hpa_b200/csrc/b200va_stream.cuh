@@ -202,4 +202,145 @@ __global__ void stream_scalar(const void* A, const void* B, void* C, size_t n, t
     if (i < n) op_elem<DT, OP>(A, B, C, i, s);
 }
 
+// ---- the grouped form: one launch over many independent (A, B, C, n) items ----------------
+// The item table and the exclusive prefix of per-item tile counts travel by value in the kernel
+// parameter block (__grid_constant__, read through the constant cache): no device allocation,
+// so a call is capturable into a CUDA graph as it stands.  One CTA per tile; a CTA finds its
+// item by binary search over the prefix, so the item index is uniform across the CTA.
+struct GroupedItem {
+    const void* a;
+    const void* b;
+    void* c;
+    size_t n;
+};
+
+template <int CAP>
+struct GroupedParams {
+    GroupedItem item[CAP];
+    unsigned long long first_tile[CAP];   // exclusive prefix of the items' tile counts
+    unsigned long long total_tiles;
+    int count;
+};
+
+// How an item is cut into tiles of `tile_vecs` 16-byte vectors.  The host (tile prefix) and the
+// device (tile body) derive it from the same pointers with this one function, exactly as the
+// stream_vec dispatcher does: `head` scalar elements up to A's 16-byte boundary, `nvec` vectors,
+// a scalar tail.  Items whose A, B and C do not share a 16-byte phase take the scalar path:
+// `tile_vecs * 16 / ES` elements per tile, one element per thread per step.  A vector item too
+// short for one vector still gets one tile: its CTA does the edge elements.
+struct GroupedShape {
+    size_t head, nvec, ntiles;
+    bool vec;
+};
+
+template <int ES, bool BINARY>
+__host__ __device__ __forceinline__ GroupedShape grouped_shape(const void* A, const void* B, const void* C, size_t n,
+                                                               size_t tile_vecs)
+{
+    const uintptr_t a = reinterpret_cast<uintptr_t>(A), b = reinterpret_cast<uintptr_t>(B), c = reinterpret_cast<uintptr_t>(C);
+    GroupedShape sh;
+    sh.vec = (a & 15u) == (c & 15u) && (!BINARY || (b & 15u) == (a & 15u));
+    if (sh.vec) {
+        sh.head = ((16u - (a & 15u)) & 15u) / ES;
+        if (sh.head > n) sh.head = n;
+        sh.nvec = (n - sh.head) * ES / 16;
+        sh.ntiles = (sh.nvec + tile_vecs - 1) / tile_vecs;
+        if (sh.ntiles == 0) sh.ntiles = 1;
+    } else {
+        const size_t tile_elems = tile_vecs * (16 / ES);
+        sh.head = 0;
+        sh.nvec = 0;
+        sh.ntiles = (n + tile_elems - 1) / tile_elems;
+    }
+    return sh;
+}
+
+// Last item whose first tile is <= tile.
+template <int CAP>
+__device__ __forceinline__ int grouped_find(const GroupedParams<CAP>& p, unsigned long long tile)
+{
+    int lo = 0, hi = p.count - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (p.first_tile[mid] <= tile) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+
+// Per element the same op_vec / op_elem as stream_vec and stream_scalar, so each item's result is
+// bit-identical to b200va_stream on it.  prefetch_first: as in stream_vec, thread 0 bulk-prefetches
+// the CTA's first tile into L2 ahead of the programmatic dependency (set for launches whose items
+// sum to >= 128 MiB per array, which cannot be L2-resident).  Every global load and store comes
+// after griddepcontrol.wait.
+template <int DT, int OP, int UNROLL, int CAP>
+__global__ void stream_grouped(const __grid_constant__ GroupedParams<CAP> p, typename dt_traits<DT>::scalar s,
+                               int prefetch_first)
+{
+    constexpr int ES = dt_traits<DT>::size;
+    constexpr int EPV = 16 / ES;
+    constexpr bool binary = (OP == OP_ADD || OP == OP_TRIAD);
+    const size_t tile_vecs = static_cast<size_t>(blockDim.x) * UNROLL;
+    pdl_launch_dependents();
+    if (prefetch_first && threadIdx.x == 0) {
+        const int i = grouped_find(p, blockIdx.x);
+        const GroupedItem& it = p.item[i];
+        const GroupedShape sh = grouped_shape<ES, binary>(it.a, it.b, it.c, it.n, tile_vecs);
+        const size_t v0 = (blockIdx.x - p.first_tile[i]) * tile_vecs;
+        if (sh.vec && v0 < sh.nvec) {
+            const uint32_t bytes = static_cast<uint32_t>((sh.nvec - v0 < tile_vecs ? sh.nvec - v0 : tile_vecs) * 16);
+            bulk_prefetch_l2(static_cast<const unsigned char*>(it.a) + sh.head * ES + v0 * 16, bytes);
+            if constexpr (binary) bulk_prefetch_l2(static_cast<const unsigned char*>(it.b) + sh.head * ES + v0 * 16, bytes);
+        }
+    }
+    pdl_wait();
+
+    for (unsigned long long tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
+        const int i = grouped_find(p, tile);
+        const GroupedItem& it = p.item[i];
+        const size_t t = tile - p.first_tile[i];
+        const GroupedShape sh = grouped_shape<ES, binary>(it.a, it.b, it.c, it.n, tile_vecs);
+        if (!sh.vec) {
+            const size_t tile_elems = tile_vecs * EPV;
+            for (size_t e = t * tile_elems + threadIdx.x; e < (t + 1) * tile_elems && e < it.n; e += blockDim.x)
+                op_elem<DT, OP>(it.a, it.b, it.c, e, s);
+            continue;
+        }
+        const unsigned char* a = static_cast<const unsigned char*>(it.a) + sh.head * ES;
+        const unsigned char* b = static_cast<const unsigned char*>(it.b) + sh.head * ES;
+        unsigned char* c = static_cast<unsigned char*>(it.c) + sh.head * ES;
+        const size_t v0 = t * tile_vecs + threadIdx.x;
+        if ((t + 1) * tile_vecs <= sh.nvec) {
+            u32x4 ra[UNROLL], rb[UNROLL];
+#pragma unroll
+            for (int j = 0; j < UNROLL; ++j) ra[j] = ldg128_bits<LD_PLAIN>(a + (v0 + static_cast<size_t>(j) * blockDim.x) * 16);
+            if constexpr (binary) {
+#pragma unroll
+                for (int j = 0; j < UNROLL; ++j) rb[j] = ldg128_bits<LD_PLAIN>(b + (v0 + static_cast<size_t>(j) * blockDim.x) * 16);
+            } else {
+#pragma unroll
+                for (int j = 0; j < UNROLL; ++j) rb[j] = u32x4{0, 0, 0, 0};
+            }
+#pragma unroll
+            for (int j = 0; j < UNROLL; ++j)
+                stg128_bits<ST_NA>(c + (v0 + static_cast<size_t>(j) * blockDim.x) * 16, op_vec<DT, OP>(ra[j], rb[j], s));
+        } else {
+#pragma unroll
+            for (int j = 0; j < UNROLL; ++j) {
+                const size_t v = v0 + static_cast<size_t>(j) * blockDim.x;
+                if (v < sh.nvec) {
+                    const u32x4 x = ldg128_bits<LD_PLAIN>(a + v * 16);
+                    const u32x4 y = binary ? ldg128_bits<LD_PLAIN>(b + v * 16) : u32x4{0, 0, 0, 0};
+                    stg128_bits<ST_NA>(c + v * 16, op_vec<DT, OP>(x, y, s));
+                }
+            }
+        }
+        if (t == 0) {
+            const size_t tail0 = sh.head + sh.nvec * EPV;
+            if (threadIdx.x < sh.head) op_elem<DT, OP>(it.a, it.b, it.c, threadIdx.x, s);
+            if (tail0 + threadIdx.x < it.n) op_elem<DT, OP>(it.a, it.b, it.c, tail0 + threadIdx.x, s);
+        }
+    }
+}
+
 }  // namespace b200va

@@ -135,6 +135,39 @@ def stream(op: str, a, b=None, out=None, *, scalar: float = 0.0, stream=None):
     return out
 
 
+def stream_grouped(op: str, a_list, b_list=None, out_list=None, *, scalar: float = 0.0, stream=None) -> list:
+    """``stream`` over many independent vectors in one b200va_stream_grouped call: item i is
+    op(a_list[i], b_list[i]) into out_list[i], bit-identical to ``stream`` on it.  Outputs are
+    allocated like ``stream`` does when ``out_list`` is None.  All tensors share one dtype and
+    one device; no output may overlap another item's tensors.  Asynchronous on the current stream."""
+    torch = _torch()
+    names = {getattr(torch, v): k for k, v in _TORCH_DT.items()}
+    a_list = list(a_list)
+    if out_list is None:
+        out_list = [torch.empty_like(a) for a in a_list]
+    out_list = list(out_list)
+    b_list = [None] * len(a_list) if b_list is None else list(b_list)
+    if not (len(a_list) == len(b_list) == len(out_list)):
+        raise TypeError("a_list, b_list and out_list differ in length")
+    if not a_list:
+        return out_list
+    dtype, device = a_list[0].dtype, a_list[0].device
+    if dtype not in names or device.type != "cuda":
+        raise TypeError("operands must be CUDA tensors of float32/float64/float16/bfloat16")
+    items = (capi.Item * len(a_list))()
+    for i, (a, b, c) in enumerate(zip(a_list, b_list, out_list)):
+        for t in (a, b, c):
+            if t is not None and (t.dtype != dtype or t.device != device or not t.is_contiguous()):
+                raise TypeError(f"item {i}: operands must be contiguous tensors of one dtype on one device")
+        if (b is not None and b.numel() != a.numel()) or c.numel() != a.numel():
+            raise TypeError(f"item {i}: operands differ in length")
+        items[i] = capi.Item(a.data_ptr(), b.data_ptr() if b is not None else None, c.data_ptr(), a.numel())
+    with torch.cuda.device(device):
+        check(lib.b200va_stream_grouped(capi.OPS[op], capi.DTYPES[names[dtype]], items, len(a_list), float(scalar),
+                                        _stream_ptr(stream)), "b200va_stream_grouped")
+    return out_list
+
+
 def probe(kind: str, a, b, c, *, stream=None):
     """Ceiling probe (b200va_probe_f32): 'read2' loads a and b, 'fill' stores c, 'copy' c = a.  c is clobbered."""
     torch = _torch()
